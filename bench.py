@@ -18,6 +18,10 @@ SynthesizerTrnMs768NSFsid.infer -> RMS mix + int16.
 Before timing, the default run checks its own output: the product path with the oracle's pitch track and noise draws against the
 fp32 CPU oracle's waveform of the same utterance (the cpu_baseline leg computes it anyway): "parity_check" in the JSON line.
 Synthetic seeded weights / audio / index (no assets, no network): "data": "synthetic".
+  --dump-outputs DIR   after the timed steps, write what the last timed step of each timed path returned as float32 .npy:
+                     device_step_audio (the device-resident step's int16 waveform) and vc_single_audio (VC.vc_single's int16
+                     waveform).  Weights, audio, index and torch's generator are seeded, so the same arguments give the same
+                     inputs on every run and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -197,7 +201,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "reference_gpu"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs is supported with --impl b200 only")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -211,6 +218,7 @@ def main():
         args.warmup = 3
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
+    torch.manual_seed(0)                 # the synthesizer's noise draws: the same on every run
     import torch.distributed as dist
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
@@ -273,7 +281,7 @@ def main():
         for s, e in ev:
             flush.fill_(1)                      # L2 flush between timed iterations (outside the event pair)
             s.record()
-            fn()
+            out = fn()
             e.record()
         torch.cuda.synchronize()
         ms = sum(s.elapsed_time(e) for s, e in ev)
@@ -281,7 +289,7 @@ def main():
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             dist.barrier()
-        return float(t.item())
+        return float(t.item()), out
 
     # the device-resident step is a fixed sequence of ~510 launches: capture it once (both streams) and replay the CUDA graph
     for _ in range(2):
@@ -305,10 +313,16 @@ def main():
     sampler = ClockSampler(local_rank)
     sampler.start()
     l0 = _lib.lib().rvcb_launch_count()
-    dev_ms = timed(step_fn, args.steps, args.warmup)
+    dev_ms, dev_out = timed(step_fn, args.steps, args.warmup)
     if not use_graph:
         launches = (_lib.lib().rvcb_launch_count() - l0) // (args.steps + args.warmup)
-    e2e_ms = timed(e2e_step, args.steps, args.warmup)
+    # copied before vc_single runs: its graphs share the model handles with the device-resident step
+    dev_out = (graph_out if use_graph else dev_out).float().cpu().numpy()
+    e2e_ms, e2e_out = timed(e2e_step, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "device_step_audio.npy"), dev_out)
+        np.save(os.path.join(args.dump_outputs, "vc_single_audio.npy"), np.asarray(e2e_out, dtype=np.float32))
     sampler.stop_flag = True
     sampler.join(timeout=2)
 
@@ -324,7 +338,7 @@ def main():
             g_full = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g_full):
                 out_full = dev_step()
-            fms = timed(g_full.replay, args.steps, args.warmup)
+            fms, _ = timed(g_full.replay, args.steps, args.warmup)
             graph.replay()
             torch.cuda.synchronize()
             same = bool(torch.equal(out_full, graph_out)) if (out_full.dtype == graph_out.dtype and out_full.shape == graph_out.shape) else None
@@ -379,7 +393,7 @@ def main():
                     cur.wait_event(e_)
             sweep = {}
             for n in conc_levels:
-                cms = timed(lambda: conc_step(n), args.steps, args.warmup)
+                cms, _ = timed(lambda: conc_step(n), args.steps, args.warmup)
                 sweep[n] = {"ms_per_step": cms / args.steps, "ms_per_utterance": cms / args.steps / n,
                             "value": world * n * args.steps * OUT_SAMPLES / (cms * 1e-3)}
             best = min(sweep, key=lambda n: sweep[n]["ms_per_utterance"])

@@ -1,6 +1,7 @@
-"""Generates tests/golden/*.npz by running the REFERENCE's own modules (imported from /root/reference in the build
-container) and, for HuBERT (un-vendored fairseq), transformers.HubertModel.  Weights/inputs come from seeds, so only the
-small outputs are stored.  Run:  python tests/golden/make_golden.py"""
+"""Generates tests/golden/*.npz by running the REFERENCE's own modules (imported from a checkout of the reference) and, for
+HuBERT (un-vendored fairseq), transformers.HubertModel.  Weights/inputs come from seeds, so only the small outputs are stored.
+Run:  python tests/golden/make_golden.py <reference checkout> [golden ...]   (no golden names: all of them)"""
+import contextlib
 import math
 import os
 import sys
@@ -9,7 +10,8 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-sys.path.insert(0, "/root/reference")
+REF = os.path.abspath(sys.argv[1])
+sys.path.insert(0, REF)
 sys.path.insert(0, ROOT)
 OUT = os.path.dirname(os.path.abspath(__file__))
 torch.set_grad_enabled(False)
@@ -18,9 +20,21 @@ torch.set_grad_enabled(False)
 from rvc.synthesizer import get_synthesizer  # noqa: E402
 from rvc.f0.e2e import E2E  # noqa: E402
 from rvc.f0.f0 import F0Predictor  # noqa: E402
-assert "/root/reference" in get_synthesizer.__code__.co_filename
+assert get_synthesizer.__code__.co_filename.startswith(REF)
 
 from oracle import weights as OW  # noqa: E402  (seeded generators only)
+
+
+@contextlib.contextmanager
+def one_thread():
+    """For goldens compared bit for bit: the float32 sums of the oracle HuBERT / RMVPE under the glue change with torch's CPU
+    thread count, so the golden and its test both run them on one thread."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(threads)
 
 
 def synth():
@@ -70,10 +84,10 @@ def rmvpe():
 
 
 def f0_fixtures():
-    z = np.load("/root/reference/infer/modules/vc/lgdsng.npz")
+    z = np.load(REF + "/infer/modules/vc/lgdsng.npz")
     np.savez_compressed(os.path.join(OUT, "ref_fixtures_f0.npz"), lgdsng_pitch=z["pitch"], lgdsng_pitchf=z["pitchf"],
-                        mute_2a_f0=np.load("/root/reference/logs/mute/2a_f0/mute.wav.npy"),
-                        mute_2b_f0nsf=np.load("/root/reference/logs/mute/2b-f0nsf/mute.wav.npy"))
+                        mute_2a_f0=np.load(REF + "/logs/mute/2a_f0/mute.wav.npy"),
+                        mute_2b_f0nsf=np.load(REF + "/logs/mute/2b-f0nsf/mute.wav.npy"))
 
 
 def hubert():
@@ -126,7 +140,7 @@ def torchgate():
         sys.modules["librosa"] = lib; sys.modules["librosa.util"] = util
     # oracle.weights put the product package (which mirrors the `infer.*` names as a regular package) on sys.path: hide it
     saved_path, saved_mods = sys.path[:], {k: sys.modules.pop(k) for k in list(sys.modules) if k == "infer" or k.startswith("infer.")}
-    sys.path[:] = ["/root/reference"] + [p for p in sys.path if "webui_b200" not in p]
+    sys.path[:] = [REF] + [p for p in sys.path if "webui_b200" not in p]
     try:
         from infer.modules.gui.torchgate import TorchGate
     finally:
@@ -134,7 +148,7 @@ def torchgate():
         for k in [k for k in sys.modules if k == "infer" or k.startswith("infer.")]:
             del sys.modules[k]
         sys.modules.update(saved_mods)
-    assert "/root/reference" in TorchGate.forward.__code__.co_filename
+    assert TorchGate.forward.__code__.co_filename.startswith(REF)
     out = {}
     # (a) the realtime GUI's instance (gui.py:869-871): sr = 48 kHz, n_fft = 4 * zc = 1920, prop_decrease 0.9, noise reference given
     x, xn = torchgate_inputs(21, 9600, 48000, 48000)
@@ -151,10 +165,10 @@ def phase_vocoder():
     """The reference's OWN phase_vocoder (gui.py:27-48).  gui.py cannot be imported (FreeSimpleGUI, sounddevice, ...): the function's
     source is cut out of the file with ast and executed with torch / numpy in scope -- the code that runs is the reference's."""
     import ast
-    src = open("/root/reference/gui.py").read()
+    src = open(REF + "/gui.py").read()
     fn = next(n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "phase_vocoder")
     ns = {"torch": torch, "np": np}
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), "/root/reference/gui.py", "exec"), ns)
+    exec(compile(ast.Module(body=[fn], type_ignores=[]), REF + "/gui.py", "exec"), ns)
     ref_pv = ns["phase_vocoder"]
     g = torch.Generator().manual_seed(77)
     out = {}
@@ -186,7 +200,7 @@ def callback_pieces():
     import types
     import torch.nn.functional as F_
     import torchaudio.transforms as tat
-    tree = ast.parse(open("/root/reference/gui.py").read())
+    tree = ast.parse(open(REF + "/gui.py").read())
     fn = next(n for n in ast.walk(tree) if isinstance(n, ast.FunctionDef) and n.name == "audio_infer")
     pv = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "phase_vocoder")
     first = next(i for i, st in enumerate(fn.body) if isinstance(st, ast.Assign) and "self.input_wav[:-self.block_frame]" in ast.unparse(st))
@@ -200,8 +214,8 @@ def callback_pieces():
                             body=list(stmts) + [ast.parse("return " + ret).body[0]], decorator_list=[])
         return ast.fix_missing_locations(ast.Module(body=[pv, f], type_ignores=[]))
     ns = {"torch": torch, "np": np, "F": F_, "sys": _sys}
-    exec(compile(make("ref_pre", ["self", "indata"], fn.body[first:gate_if + 1], "None"), "/root/reference/gui.py", "exec"), ns)
-    exec(compile(make("ref_sola", ["self", "infer_wav"], fn.body[sola0:sola1 + 1], "infer_wav, sola_offset"), "/root/reference/gui.py", "exec"), ns)
+    exec(compile(make("ref_pre", ["self", "indata"], fn.body[first:gate_if + 1], "None"), REF + "/gui.py", "exec"), ns)
+    exec(compile(make("ref_sola", ["self", "infer_wav"], fn.body[sola0:sola1 + 1], "infer_wav, sola_offset"), REF + "/gui.py", "exec"), ns)
     # the reference's TorchGate (same import trick as torchgate())
     if "librosa" not in sys.modules:
         lib = types.ModuleType("librosa"); util = types.ModuleType("librosa.util")
@@ -209,7 +223,7 @@ def callback_pieces():
         lib.util = util
         sys.modules["librosa"] = lib; sys.modules["librosa.util"] = util
     saved_path, saved_mods = sys.path[:], {k: sys.modules.pop(k) for k in list(sys.modules) if k == "infer" or k.startswith("infer.")}
-    sys.path[:] = ["/root/reference"] + [p for p in sys.path if "webui_b200" not in p]
+    sys.path[:] = [REF] + [p for p in sys.path if "webui_b200" not in p]
     try:
         from infer.modules.gui.torchgate import TorchGate
     finally:
@@ -249,6 +263,7 @@ def callback_pieces():
     np.savez_compressed(os.path.join(OUT, "callback_pieces.npz"), **out)
 
 
+@one_thread()
 def vc_glue():
     """The reference's OWN ``Pipeline.vc`` (infer/modules/vc/pipeline.py:76-184), cut out of the file with ast (the module itself needs
     faiss / librosa to import) and executed with duck-typed components: ``model`` = the oracle HuBERT (so only the glue is under test),
@@ -259,11 +274,11 @@ def vc_glue():
     from time import time as _time
     import torch.nn.functional as F_
     from oracle import hubert as OH, ivf as OI
-    tree = ast.parse(open("/root/reference/infer/modules/vc/pipeline.py").read())
+    tree = ast.parse(open(REF + "/infer/modules/vc/pipeline.py").read())
     cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "Pipeline")
     vc = next(n for n in cls.body if isinstance(n, ast.FunctionDef) and n.name == "vc")
     ns = {"torch": torch, "np": np, "F": F_, "time": _time}
-    exec(compile(ast.fix_missing_locations(ast.Module(body=[vc], type_ignores=[])), "/root/reference/infer/modules/vc/pipeline.py", "exec"), ns)
+    exec(compile(ast.fix_missing_locations(ast.Module(body=[vc], type_ignores=[])), REF + "/infer/modules/vc/pipeline.py", "exec"), ns)
     ref_vc = ns["vc"]
     hw = OW.hubert_weights(777)
 
@@ -317,13 +332,13 @@ def pipeline_flow():
     import types
     from time import time as _time
     from scipy import signal
-    tree = ast.parse(open("/root/reference/infer/modules/vc/pipeline.py").read())
+    tree = ast.parse(open(REF + "/infer/modules/vc/pipeline.py").read())
     cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "Pipeline")
     fn = next(n for n in cls.body if isinstance(n, ast.FunctionDef) and n.name == "pipeline")
     bh, ah = signal.butter(N=5, Wn=48, btype="high", fs=16000)                 # pipeline.py:23
     ns = {"torch": torch, "np": np, "os": os, "signal": signal, "time": _time, "bh": bh, "ah": ah,
           "traceback": __import__("traceback")}
-    exec(compile(ast.fix_missing_locations(ast.Module(body=[fn], type_ignores=[])), "/root/reference/infer/modules/vc/pipeline.py", "exec"), ns)
+    exec(compile(ast.fix_missing_locations(ast.Module(body=[fn], type_ignores=[])), REF + "/infer/modules/vc/pipeline.py", "exec"), ns)
     sr, tgt_sr, x_pad, x_query, x_center, x_max = 16000, 1600, 1, 1, 3, 4
     me = types.SimpleNamespace(window=160, sr=sr, device="cpu", t_pad=sr * x_pad, t_pad_tgt=tgt_sr * x_pad, t_pad2=sr * x_pad * 2,
                                t_query=sr * x_query, t_center=sr * x_center, t_max=sr * x_max)
@@ -339,6 +354,7 @@ def pipeline_flow():
                         total=np.float64(np.abs(out.astype(np.float64)).sum()), out_nof0=out0[::3].astype(np.float32), n_nof0=np.int64(out0.shape[0]))
 
 
+@one_thread()
 def rtrvc_glue():
     """The reference's OWN realtime ``RVC.infer`` (infer/lib/rtrvc.py:134-260), cut out with ast (the module needs fairseq / faiss to
     import) and run on a stand-in ``self``: hubert = the oracle HuBERT, index = the oracle IVF-Flat object, ``_get_f0`` = the oracle RMVPE
@@ -351,11 +367,11 @@ def rtrvc_glue():
     from typing import Union, Optional, Literal
     from torchaudio.transforms import Resample
     from oracle import hubert as OH, ivf as OI, rmvpe as ORM
-    tree = ast.parse(open("/root/reference/infer/lib/rtrvc.py").read())
+    tree = ast.parse(open(REF + "/infer/lib/rtrvc.py").read())
     cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "RVC")
     fns = [n for n in cls.body if isinstance(n, ast.FunctionDef) and n.name in ("infer", "_get_f0")]
     ns = {"torch": torch, "np": np, "F": F_, "Union": Union, "Optional": Optional, "Literal": Literal, "Resample": Resample}
-    exec(compile(ast.fix_missing_locations(ast.Module(body=fns, type_ignores=[])), "/root/reference/infer/lib/rtrvc.py", "exec"), ns)
+    exec(compile(ast.fix_missing_locations(ast.Module(body=fns, type_ignores=[])), REF + "/infer/lib/rtrvc.py", "exec"), ns)
     hw, rw = OW.hubert_weights(777), OW.rmvpe_weights(4321)
 
     class Model:
@@ -401,13 +417,13 @@ def rmvpe_compute_f0():
     import torch.nn.functional as F_
     from typing import Optional, Union
     from oracle import rmvpe as ORM
-    tree = ast.parse(open("/root/reference/rvc/f0/rmvpe.py").read())
+    tree = ast.parse(open(REF + "/rvc/f0/rmvpe.py").read())
     cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "RMVPE")
     want = ("compute_f0", "_mel2hidden", "_decode", "_to_local_average_cents")
     fns = [n for n in cls.body if isinstance(n, ast.FunctionDef) and n.name in want]
     assert len(fns) == len(want)
     ns = {"torch": torch, "np": np, "F": F_, "Optional": Optional, "Union": Union}
-    exec(compile(ast.fix_missing_locations(ast.Module(body=fns, type_ignores=[])), "/root/reference/rvc/f0/rmvpe.py", "exec"), ns)
+    exec(compile(ast.fix_missing_locations(ast.Module(body=fns, type_ignores=[])), REF + "/rvc/f0/rmvpe.py", "exec"), ns)
     Stand = type("Stand", (F0Predictor,), {k: ns[k] for k in want})
     me = Stand(160, 30, 8000, 16000, "cpu")
     me.is_half = False
@@ -424,8 +440,53 @@ def rmvpe_compute_f0():
     np.savez_compressed(os.path.join(OUT, "rmvpe_compute_f0.npz"), **out)
 
 
+def reference_modules(stride=7):
+    """The reference's OWN synthesizer classes (rvc/synthesizer.py: the v2/48k f0 model, its realtime skip_head / return_length
+    path, the no-f0 family and the v1/48k, v1/32k, v2/32k decoder schedules) and RMVPE network (rvc/f0/e2e.py) on seeded weights,
+    inputs and noise, with each model's state-dict key set.  Outputs are stored every ``stride``-th value (7 is coprime with the
+    480 / 320 up-sampling and the 360 salience bins); tests/test_oracle_vs_reference.py draws the same inputs in the same order."""
+    g = torch.Generator().manual_seed(1)
+    T = 60
+    phone = torch.randn(1, T, 768, generator=g) * 0.5
+    pitchf = torch.zeros(1, T); pitchf[:, 5:50] = 150 + 50 * torch.rand(45, generator=g)
+    fm = 1127 * torch.log(1 + pitchf / 700); mn, mx = 1127 * math.log(1 + 50 / 700), 1127 * math.log(1 + 1100 / 700)
+    pitch = torch.round(torch.where(fm > 0, (fm - mn) * 254 / (mx - mn) + 1, fm).clamp(1, 255)).long()
+    out = {"stride": np.int64(stride)}
+
+    def model(name, cpt):
+        net, _ = get_synthesizer({**cpt, "weight": dict(cpt["weight"]), "config": list(cpt["config"])}, "cpu")
+        out[name + "_keys"] = np.array(sorted(net.state_dict()))
+        return net
+
+    def keep(name, y):
+        out[name], out[name + "_shape"] = y.numpy().reshape(-1)[::stride].copy(), np.array(y.shape, dtype=np.int64)
+    net_g = model("v2_48k", OW.synth_cpt(77, "v2"))
+    torch.manual_seed(5); keep("v2_48k", net_g.infer(phone, torch.tensor([T]), torch.tensor([2]), pitch, pitchf))
+    torch.manual_seed(6)
+    keep("v2_48k_rt", net_g.infer(phone, torch.tensor([T]), torch.tensor([2]), pitch, pitchf, skip_head=40, return_length=12, return_length2=14))
+    net0 = model("nof0", OW.synth_cpt(5, "v2", f0=0))
+    torch.manual_seed(3); keep("nof0", net0.infer(phone, torch.tensor([T]), torch.tensor([1])))
+    for name, cfgx, ver in (("v1_48k", OW.V1_48K_CONFIG, "v1"), ("v1_32k", OW.V1_32K_CONFIG, "v1"), ("v2_32k", OW.V2_32K_CONFIG, "v2")):
+        netx = model(name, OW.synth_cpt(5, ver, config=cfgx))
+        Tx = 24; phx = torch.randn(1, Tx, 256 if ver == "v1" else 768, generator=g) * 0.5
+        torch.manual_seed(3); keep(name, netx.infer(phx, torch.tensor([Tx]), torch.tensor([1]), pitch[:, :Tx], pitchf[:, :Tx]))
+    m = E2E(4, 1, (2, 2)).eval()
+    out["e2e_keys"] = np.array(sorted(m.state_dict()))
+    m.load_state_dict(OW.rmvpe_weights(9))
+    keep("e2e", m(torch.randn(1, 128, 96, generator=g) * 3 - 4))
+    np.savez_compressed(os.path.join(OUT, "reference_modules.npz"), **out)
+
+
+GOLDENS = (synth, rmvpe, f0_fixtures, hubert, torchgate, phase_vocoder, callback_pieces, vc_glue, pipeline_flow, rtrvc_glue,
+           rmvpe_compute_f0, reference_modules)
+
 if __name__ == "__main__":
-    synth(); rmvpe(); f0_fixtures(); hubert(); torchgate(); phase_vocoder(); callback_pieces(); vc_glue(); pipeline_flow(); rtrvc_glue()
-    rmvpe_compute_f0()
+    names = sys.argv[2:] or [fn.__name__ for fn in GOLDENS]
+    unknown = set(names) - {fn.__name__ for fn in GOLDENS}
+    if unknown:
+        sys.exit(f"unknown golden(s) {sorted(unknown)}; choose from {[fn.__name__ for fn in GOLDENS]}")
+    for fn in GOLDENS:
+        if fn.__name__ in names:
+            fn()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))

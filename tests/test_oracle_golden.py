@@ -1,5 +1,6 @@
 """CPU: the oracle against golden vectors produced by the REFERENCE's own modules (tests/golden/make_golden.py) and the
 reference's own fixtures (infer/modules/vc/lgdsng.npz, logs/mute/2a_f0, 2b-f0nsf)."""
+import contextlib
 import math
 import os
 
@@ -7,6 +8,17 @@ import numpy as np
 import torch
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+@contextlib.contextmanager
+def one_thread():
+    """As tests/golden/make_golden.py::one_thread made the glue goldens: the oracle's float32 sums depend on the thread count."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(threads)
 
 
 def test_synth_oracle_matches_reference_golden():
@@ -172,6 +184,7 @@ def test_callback_oracle_matches_the_reference_statements():
         assert len(set(offs)) > 1
 
 
+@one_thread()
 def test_pipeline_vc_glue_oracle_matches_the_reference_method():
     """oracle.pipeline.OraclePipeline.vc vs what the reference's OWN ``Pipeline.vc`` (pipeline.py:76-184, executed from its source on
     duck-typed components by tests/golden/make_golden.py::vc_glue) hands to the synthesizer: retrieval weights + blend, x2 nearest
@@ -233,6 +246,7 @@ def test_pipeline_control_flow_oracle_matches_the_reference_method():
     assert out0.shape[0] == int(z["n_nof0"]) and np.array_equal(out0[::3].astype(np.float32), z["out_nof0"])
 
 
+@one_thread()
 def test_rtrvc_oracle_matches_the_reference_method():
     """oracle.rtrvc.OracleRVC.infer vs the reference's OWN realtime ``RVC.infer`` (infer/lib/rtrvc.py:134-260, executed from its source
     on duck-typed components by tests/golden/make_golden.py::rtrvc_glue) over three consecutive rolling-window blocks: what reaches the
